@@ -16,6 +16,8 @@ steps are software-pipelined (the encode of batch k+1 runs beside the latency-bo
 batches); the strictly sequential figures are reported beside them (`sequential`,
 `e2e.sequential_value`) and `--no-pipeline` makes them the headline.  Timing: CUDA events on the stream
 all work forks from and joins, barrier + synchronize on both sides, max over ranks.
+`--dump-outputs DIR` also writes what the last timed step computed as DIR/<name>.npy; the inputs are seeded, so
+two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -34,6 +36,8 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 METRIC = 'Mpixels/s encode+decode (lossless round-trip)'
+# --dump-outputs: elements per array (16 MB as float32), so that a dump stays far below 64 MB
+DUMP_MAX_ELEMENTS = 1 << 22
 
 # conv FLOPs per pixel of a round trip (SURVEY.md 8d): encode forward + decoder-side re-run
 WORKLOADS = {
@@ -297,7 +301,7 @@ def run_ours(args):
     def step_resident(imgs):
         blob, info = codec.encode_batch(imgs, pad_tuple, to_host=False, tile=TILE['v'])
         S = codec.decode_device(blob, info['stream_offsets'], info['lens'], shapes_of(info), tile=TILE['v'])
-        return S, info
+        return S, info, blob
 
     tmpdir = None
     if crops_mode:
@@ -338,8 +342,8 @@ def run_ours(args):
     def run_resident(steps, first_set=0):
         if not args.pipeline:
             for s in range(steps):
-                S, info = step_resident(dev_sets[(first_set + s) % n_sets])
-            return S, info
+                S, info, blob = step_resident(dev_sets[(first_set + s) % n_sets])
+            return S, info, blob
         dbg = os.environ.get('L3C_BENCH_DEBUG')
         cur = torch.cuda.current_stream()
         for es in enc_streams:
@@ -414,7 +418,7 @@ def run_ours(args):
                     line += '  stages: ' + ' '.join('%s=%.1f' % (n2, e1.elapsed_time(e2))
                                                      for (_, e1), (n2, e2) in zip(evs[:-1], evs[1:]))
                 print(line, file=sys.stderr)
-        return S, info
+        return S, info, blob
 
     def run_e2e(steps, first_set=0):
         if not args.pipeline or crops_mode:
@@ -470,13 +474,36 @@ def run_ours(args):
                 parts = [l3c_pad.undo_pad(S[i * per + j:i * per + j + 1], *pad_tuple) for j in range(per)]
                 assert torch.equal(auto_crop.stitch(parts)[0].cpu(), raw_sets[k][i]), what + ': stitched image differs'
 
+    def dump_outputs(out_dir, S, info, blob):
+        """What the last timed step handed its caller, as out_dir/<name>.npy: the decoded images, the coded
+        bytes of every stream (container order, concatenated), the container sizes and the stream lengths.
+        An array of more than DUMP_MAX_ELEMENTS elements is cut to a fixed, seeded sample of its elements."""
+        def sample(n):
+            if n <= DUMP_MAX_ELEMENTS:
+                return np.arange(n, dtype=np.int64)
+            return np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ELEMENTS, replace=False))
+
+        lens = np.asarray(info['lens'], np.int64).reshape(-1)
+        ends = np.cumsum(lens)
+        pos = sample(int(ends[-1]))                       # positions in the concatenated streams
+        j = np.searchsorted(ends, pos, side='right')
+        at = np.asarray(info['stream_offsets'], np.int64).reshape(-1)[j] + pos - (ends[j] - lens[j])
+        arrays = {'decoded': S.reshape(-1)[torch.from_numpy(sample(S.numel())).to(dev)],
+                  'streams': blob[torch.from_numpy(at).to(dev)]}
+        arrays = {k: v.cpu().numpy().astype(np.float32) for k, v in arrays.items()}
+        arrays['container_bytes'] = np.asarray(info['sizes'], np.float64)
+        arrays['stream_lens'] = np.asarray(info['lens'], np.float64)
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + '.npy'), a)
+
     # ---- warm-up + correctness (outside the timed region)
     for w in range(max(args.warmup, 1)):
-        S, info = step_resident(dev_sets[w % n_sets])
+        S, info, _ = step_resident(dev_sets[w % n_sets])
     check_lossless(S, (max(args.warmup, 1) - 1) % n_sets, 'warm-up')
     if args.pipeline:                      # every lane / encode stream has its own allocator pool: warm them all up
         n_warm = max(args.warmup, n_lanes + 1)     # (a first use inside the timed region costs a 300 ms cudaMalloc stall)
-        S, info = run_resident(n_warm)
+        S, info, _ = run_resident(n_warm)
         check_lossless(S, (n_warm - 1) % n_sets, 'pipelined warm-up')
     sizes = info['sizes']
     counts = l3c_dist.gather_byte_counts(sizes, n_global * (n_units // n_img), rank, world)   # the one collective
@@ -510,7 +537,7 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     launches0 = E.LAUNCHES['n']
-    S, info = run_resident(args.steps)
+    S, info, blob = run_resident(args.steps)
     launches_timed = E.LAUNCHES['n'] - launches0
     e1.record()
     barrier()
@@ -522,6 +549,8 @@ def run_ours(args):
     ms_total = float(ms)
     value = px_step_global * args.steps / 1e6 / (ms_total / 1e3)
     check_lossless(S, (args.steps - 1) % n_sets, 'timed run')
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, S, info, blob)
 
     def timed_sequential(fn):
         """the same K steps strictly one after the other (reported beside the pipelined numbers)"""
@@ -559,7 +588,7 @@ def run_ours(args):
     if not crops_mode and TILE['v'] is None and not args.no_tiled:
         TILE['v'] = (64, 64)
         try:
-            S, info_t = step_resident(dev_sets[0])
+            S, info_t, _ = step_resident(dev_sets[0])
             check_lossless(S, 0, 'tiled')
             t_seq, _ = timed_sequential(lambda i: step_resident(dev_sets[i]))
             t_pipe = None
@@ -568,7 +597,7 @@ def run_ours(args):
                 barrier()
                 a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 a.record()
-                S, _ = run_resident(args.steps)
+                S, _, _ = run_resident(args.steps)
                 b.record()
                 barrier()
                 t_pipe = a.elapsed_time(b)
@@ -828,6 +857,9 @@ def main():
                     help='decodes in flight in the pipelined mode (default: 4; rgb_shared: 1)')
     ap.add_argument('--no-pipeline', dest='pipeline', action='store_false',
                     help='strictly sequential steps: encode(k), decode(k), encode(k+1), ...')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed (rank 0) as DIR/<name>.npy, float32/float64, '
+                         'to compare two builds output for output')
     args = ap.parse_args()
     if args.impl == 'reference':
         return run_reference(args)
